@@ -8,8 +8,13 @@ argmin + top-10 (selection fused into the kernel's epilogue, no acq[M] materiali
 `--config c5` = BASELINE configs[4]: d=32, N_train=8192, UCB, 2^22 candidates in TOTAL sharded over the
 ranks (strong scaling), NCCL all-gather of the per-rank records for the final argmax.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3|c5] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3|c5] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes, as float64 .npy, the merged selection records of the LAST timed device step
+(device_argmin_index, device_argmin_value, device_top_indices) and, on one rank, what the last timed
+FusedAcquisition.argmin_topk call returned (e2e_*).  The inputs depend only on the arguments (fixed seeds), so two
+builds can be compared output for output.
 
 Keys beyond the base contract:
   value         candidates already resident in HBM (device entry point of the C ABI), whole job
@@ -43,14 +48,10 @@ import time  # noqa: E402
 
 import numpy as np  # noqa: E402
 
-# the reference package: vendored unmodified by tools/vendor_ref.py (git-ignored oracle/_ref, ships with gpurun)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-try:
-    import vendor_ref
+# the reference package: vendored unmodified by build() (oracle/vendor_ref.py, git-ignored oracle/_ref); only read here
+from oracle.vendor_ref import ref_dir  # noqa: E402
 
-    _REF_DIR = vendor_ref.vendor()
-except Exception:  # pragma: no cover
-    _REF_DIR = None
+_REF_DIR = ref_dir()
 if _REF_DIR and _REF_DIR not in sys.path:
     sys.path.insert(0, _REF_DIR)
 
@@ -201,8 +202,8 @@ def run_reference(args, rank, world):
         return
     cfg = CONFIGS[args.config]
     if _REF_DIR is None:
-        emit({"impl": "reference", "unavailable": "oracle/_ref (vendored bayes_opt) is missing: run tools/vendor_ref.py "
-                                                  "where /root/reference exists"})
+        emit({"impl": "reference", "unavailable": "oracle/_ref (vendored bayes_opt) is missing: build() runs "
+                                                  "oracle/vendor_ref.py where the reference source tree is present"})
         return
     import threadpoolctl
 
@@ -249,6 +250,13 @@ def emit(line):
     out.flush()
 
 
+def dump_outputs(path, arrays):
+    """Each array as path/<name>.npy in float64 (row indices are exact in float64 below 2^53)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def ncu_traffic(kernel):
     """dram bytes per launch of `kernel` from this round's committed ncu capture (profiles/r02_ncu_traffic.json,
     written by tools/ncu_summary.py from the .ncu-rep), or None."""
@@ -269,6 +277,7 @@ def main():
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary legs (fp32, throughput, c5, fit, suggest)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -394,6 +403,8 @@ def main():
 
         total_ms, kernel_ms, launches, clocks = timed(step_device, steps, warmup, sample_clocks)
         m_step = world * m_local if cfg["scaling"] == "weak" else cfg["m_total"]
+        last = merged_result(sel, gathered)  # what the last timed step computed
+        outputs = {"device_argmin_index": last[0], "device_argmin_value": last[1], "device_top_indices": last[2]}
         step_device(0)  # untimed: the reported result is always that of candidate buffer 0 (comparable across legs / N)
         res = merged_result(sel, gathered)
         out = {"value": m_step * steps / (total_ms * 1e-3), "ms_per_step": total_ms / steps, "kernel_ms": float(np.mean(kernel_ms)),
@@ -422,6 +433,8 @@ def main():
                 # candidates in, (argmin, value, seed indices) out.  Inside: finite check, chunked H2D overlapped with
                 # the fused kernel + selection, D2H of the records.
                 idx, val, top = acq.argmin_topk(host_np[i % N_CAND_BUFFERS], KSEEDS)
+                if world == 1:  # with more ranks this is one shard's result, not the job's
+                    outputs.update(e2e_argmin_index=idx, e2e_argmin_value=val, e2e_top_indices=top)
                 if world > 1:  # the exchange step, from host-side records
                     rec = torch.full((KSEEDS + 1, 2), -1, dtype=torch.int64)
                     rec[0, 0] = int(np.float64(val).view(np.int64))
@@ -436,11 +449,14 @@ def main():
                           "api": "FusedAcquisition.argmin_topk(host ndarray (pageable), k) - the package's public call: finite "
                                  "check, H2D of the batch in chunks overlapped with the fused kernel + selection, D2H of the records"}
         out["_keep"] = (gp, acq, dev_bufs, host_bufs, X, y)
+        out["_outputs"] = outputs
         return out
 
     cfg = CONFIGS[args.config]
     main_leg = run_config(cfg, args.steps, args.warmup)
     gp, acq, dev_bufs, host_bufs, X, y = main_leg.pop("_keep")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main_leg.pop("_outputs"))
     extra = {}
 
     if not args.no_extra and args.config == "c3":

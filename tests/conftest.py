@@ -9,16 +9,12 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
-# The reference package (bayes_opt) drives the drop-in tests.  It is vendored, unmodified, into the
-# git-ignored oracle/_ref by tools/vendor_ref.py (here, where /root/reference exists) and travels to the GPU
-# box with the snapshot; the product package imports `bayes_opt` from sys.path like any user environment.
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-try:
-    import vendor_ref
+# The reference package (bayes_opt) drives the drop-in tests.  build() vendors it, unmodified, into the
+# git-ignored oracle/_ref (oracle/vendor_ref.py), which stays with the built tree; the tests only read it.  The
+# product package imports `bayes_opt` from sys.path like any user environment.
+from oracle.vendor_ref import ref_dir  # noqa: E402
 
-    _REF = vendor_ref.vendor()
-except Exception:  # pragma: no cover
-    _REF = None
+_REF = ref_dir()
 if _REF and _REF not in sys.path:
     sys.path.insert(0, _REF)
 
@@ -43,8 +39,8 @@ def _skip_without_reference(items):
         pass
     import inspect
 
-    skip = pytest.mark.skip(reason="bayes_opt not importable: run tools/vendor_ref.py where /root/reference exists "
-                                   "(oracle/_ref ships with the repository snapshot)")
+    skip = pytest.mark.skip(reason="bayes_opt not importable: build() vendors it into oracle/_ref "
+                                   "(oracle/vendor_ref.py) where the reference source tree is present")
     for item in items:
         try:
             src = inspect.getsource(item.function)
@@ -90,5 +86,5 @@ def ref():
     try:
         import bayes_opt
     except ImportError:
-        pytest.skip("reference package bayes_opt not importable (run tools/vendor_ref.py where /root/reference exists)")
+        pytest.skip("reference package bayes_opt not importable (build() vendors it with oracle/vendor_ref.py)")
     return bayes_opt

@@ -2,7 +2,7 @@
 
     python -m pytest -p tests.ref_suite_plugin oracle/_ref/ref_tests
 
-The reference's tests (vendored, unmodified, into the git-ignored oracle/_ref/ref_tests by tools/vendor_ref.py)
+The reference's tests (vendored, unmodified, into the git-ignored oracle/_ref/ref_tests by oracle/vendor_ref.py)
 build their objects from three names: ``sklearn.gaussian_process.GaussianProcessRegressor``, the classes of
 ``bayes_opt.acquisition`` and ``bayes_opt.constraint.ConstraintModel``.  Before those modules are collected this
 plugin rebinds the names to the B200 classes (which ARE the reference's classes + the device hooks), so every

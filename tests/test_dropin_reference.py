@@ -1,4 +1,4 @@
-"""Drop-in mechanics against the REAL reference package (vendored, unmodified: tools/vendor_ref.py).
+"""Drop-in mechanics against the REAL reference package (vendored, unmodified: oracle/vendor_ref.py).
 No device work here: checks that ``enable`` swaps the three seams, that the hooked objects ARE the
 reference's objects (state and types kept), and that the product package restates nothing of them.
 The device-side behaviour of the same objects is tests/test_gpu_dropin_live.py."""

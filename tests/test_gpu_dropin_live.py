@@ -9,7 +9,7 @@ suggest()/register() side by side (R/bayes_opt/bayesian_optimization.py:323-333,
     reference's under the REFERENCE's own acquisition closure (sklearn/scipy on the host).
 
 Both optimizers then register the reference's point, so the trajectories stay comparable.  The vendored
-package (oracle/_ref, tools/vendor_ref.py) is the unmodified reference."""
+package (oracle/_ref, oracle/vendor_ref.py) is the unmodified reference."""
 import warnings
 
 import numpy as np

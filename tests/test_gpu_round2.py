@@ -356,3 +356,29 @@ def test_white_kernel_term_vs_sklearn(bo, order):
     assert r1.uniform() == r0.uniform()
     assert gpf.log_marginal_likelihood_value_ == pytest.approx(skf.log_marginal_likelihood_value_, rel=1e-6, abs=1e-6)
     assert_allclose(gpf.kernel_.theta, skf.kernel_.theta, rtol=0, atol=5e-3)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: with one timed step (warm-up >= 3 rotates back to candidate buffer 0) the dumped device
+    records are the step whose result the JSON line reports; every file is float64."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "1", "--warmup", "3",
+                          "--no-extra", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-3000:]
+    j = json.loads(out.stdout.strip().splitlines()[-1])
+    assert j["steps"] == 1
+    d = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(d) == sorted(f"{leg}_{name}" for leg in ("device", "e2e")
+                               for name in ("argmin_index", "argmin_value", "top_indices"))
+    assert all(a.dtype == np.float64 for a in d.values())
+    r = j["result"]
+    assert int(d["device_argmin_index"]) == r["argmin_index"]
+    assert_allclose(float(d["device_argmin_value"]), r["argmin_value"], rtol=1e-12, atol=0)
+    assert [int(t) for t in d["device_top_indices"]] == r["top_indices"]
+    assert d["e2e_top_indices"].shape == (10,)

@@ -15,15 +15,17 @@ SUITE = os.path.join(ROOT, "oracle", "_ref", "ref_tests")
 
 def run_reference_suite(extra=()):
     env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "tests") + os.pathsep + os.environ.get("PYTHONPATH", ""))
+    # --confcutdir: with `-c /dev/null` pytest would otherwise collect every parent directory of the suite up to
+    # the filesystem root, and fail on one the user may not list.
     cmd = [sys.executable, "-m", "pytest", "-q", "-p", "ref_suite_plugin", "-p", "no:cacheprovider", "--tb=line",
-           "-c", os.devnull, "--rootdir", SUITE, SUITE, *extra]
+           "-c", os.devnull, "--rootdir", SUITE, "--confcutdir", SUITE, SUITE, *extra]
     return subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=1500)
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="GPU present: tests/test_gpu_reference_suite.py runs the suite")
 def test_reference_suite_without_gpu_fails_only_with_the_loud_device_error():
     if not os.path.isdir(SUITE):
-        pytest.skip("reference tests not vendored (tools/vendor_ref.py needs /root/reference)")
+        pytest.skip("reference tests not vendored (build() runs oracle/vendor_ref.py where the reference is present)")
     out = run_reference_suite().stdout
     m = re.search(r"(\d+) failed, (\d+) passed", out)
     assert m, out[-2000:]

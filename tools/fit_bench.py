@@ -11,7 +11,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))  # the vendored, unmodified reference (tools/vendor_ref.py)
+sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))  # the vendored, unmodified reference (oracle/vendor_ref.py)
 import bayesianoptimization_b200 as bo  # noqa: E402
 from bayes_opt.target_space import TargetSpace  # noqa: E402
 from sklearn.gaussian_process.kernels import Matern  # noqa: E402
