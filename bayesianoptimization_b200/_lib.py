@@ -26,7 +26,7 @@ EXPORTS = [
     "b200bo_gp_set_transform", "b200bo_gp_fit",
     "b200bo_gp_set_data", "b200bo_gp_append", "b200bo_gp_lml", "b200bo_gp_get", "b200bo_gp_n", "b200bo_gp_dim",
     "b200bo_gp_predict", "b200bo_gp_predict_cov", "b200bo_acq_eval", "b200bo_acq_argmin_topk", "b200bo_acq_eval_dev",
-    "b200bo_last_kernel_ms",
+    "b200bo_last_kernel_ms", "b200bo_last_select_stats",
     "b200bo_acq_argmin_topk_philox", "b200bo_acq_select_philox_dev", "b200bo_philox_rows",
     "b200bo_gp_replicate", "b200bo_multi_gpu_acq_argmin_topk", "b200bo_multi_gpu_acq_argmin_topk_philox",
     "b200bo_multi_gpu_acq_eval",
@@ -99,6 +99,7 @@ def lib():
                                       C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int64,
                                       C.c_void_p]
     L.b200bo_last_kernel_ms.argtypes = [C.POINTER(C.c_float)]
+    L.b200bo_last_select_stats.argtypes = [i64p, i64p]
     philox_outs = [dp, i64p, dp, dp, i64p, dp]
     L.b200bo_acq_argmin_topk_philox.argtypes = [C.POINTER(AcqSpec), C.c_uint64, dp, dp, C.c_int64, C.c_int64,
                                                 C.c_int, *philox_outs]

@@ -112,6 +112,11 @@ struct b200bo_gp {
     bool tc_valid = false;
     DevBuf cov_xc, cov_kst, cov_v, cov_c, cov_out, cov_mu;  // predict(return_cov=True) scratch
     DevBuf sel_cta;         // per-CTA running selection lists of the fused kernels
+    // pruned selection: screen keys [m], survivors / pilot (coordinates + global index), counters
+    // ([0] survivors, [1] pilot candidates, [2] tau); work of the last call for b200bo_last_select_stats
+    DevBuf prune_key, surv, pilot, prune_cnt;
+    long long st_screened = 0, st_full = 0;
+    bool st_pruned = false;
     DevBuf pbounds, prow;   // throughput mode: Philox bounds (lo, span) / regenerated winner rows
     bool replica = false;   // predict-only copy made by b200bo_gp_replicate
     // look-ahead Cholesky: bulk stream, chain/bulk events, copy of the next diagonal step's panel block
@@ -204,8 +209,12 @@ static int init_handle(b200bo_gp* gp) {
     CU(cudaFuncSetAttribute(predict_acq_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesTc3));
     CU(cudaFuncSetAttribute(predict_acq_tc4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesTc4));
     CU(cudaFuncSetAttribute(small_trsv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmallTrsvSmemBytes));
-    CU(cudaFuncSetAttribute(predict_acq16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
-    CU(cudaFuncSetAttribute(predict_acq16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<true, P16_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<false, P16_FULL>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<true, P16_SCREEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<false, P16_SCREEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<true, P16_GATHER>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
+    CU(cudaFuncSetAttribute(predict_acq16_kernel<false, P16_GATHER>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPredictSmemBytesDmma));
     CU(cudaFuncSetAttribute(trailing_update64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTrailSmemBytes));
     CU(cudaFuncSetAttribute(dgemm128_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemm128SmemBytes));
     CU(cudaFuncSetAttribute(dgemm128_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemm128SmemBytes));
@@ -244,7 +253,8 @@ extern "C" void b200bo_gp_destroy(b200bo_gp* gp) {
                       &gp->pscratch, &gp->xc, &gp->out_acq, &gp->out_mu, &gp->out_sd, &gp->sel,
                       &gp->clamp, &gp->s_ksm, &gp->s_partial, &gp->s_mupart, &gp->s_unit, &gp->s_rb, &gp->s_colsq,
                       &gp->tc_linv, &gp->cov_xc, &gp->cov_kst, &gp->cov_v, &gp->cov_c, &gp->cov_out, &gp->cov_mu,
-                      &gp->sel_cta, &gp->pbounds, &gp->prow, &gp->pside};
+                      &gp->sel_cta, &gp->pbounds, &gp->prow, &gp->pside, &gp->prune_key, &gp->surv, &gp->pilot,
+                      &gp->prune_cnt};
     for (DevBuf* b : bufs) b->release();
     if (gp->stream) cudaStreamDestroy(gp->stream);
     if (gp->fgraph_exec) cudaGraphExecDestroy(gp->fgraph_exec);
@@ -1021,10 +1031,85 @@ struct CandSrc {
 
 // resume != 0: the per-CTA selection lists of the previous launch on this handle are continued instead of
 // re-initialised (chunked batches: one merge after the last chunk); finish == 0 skips the merge.
+// m_call: candidates of the whole chunked call (0: this launch's m).
 struct SelMode {
     int resume = 0;
     int finish = 1;
+    long long m_call = 0;
 };
+
+template <int MODE>
+static void launch16(bool dreg, int grid, const PredictParams& P, cudaStream_t stream) {
+    if (dreg)
+        predict_acq16_kernel<true, MODE><<<grid, P16_NT, kPredictSmemBytesDmma, stream>>>(P);
+    else
+        predict_acq16_kernel<false, MODE><<<grid, P16_NT, kPredictSmemBytesDmma, stream>>>(P);
+    LAUNCHED();
+}
+
+// Pruned selection (DESIGN.md 4.1): whether a fused-selection call takes it.  The acquisition must grow with
+// sigma; the records alone are asked for; the screen (phase A + kScreenBlocks row blocks per candidate) must be
+// a small part of the full product (np >= 8 row blocks); and the batch must span enough waves of tiles to repay
+// the two full-tile latencies of the pilot and the survivor launch (measured, DESIGN.md 6).
+constexpr int kPruneMinBlocks = 8;
+constexpr long long kPruneMinWaves = 4;
+
+static bool prune_eligible(const b200bo_acq* spec, long long m_call, int np_max, int sm_count) {
+    const bool monotone = spec->kind == B200BO_ACQ_EI || spec->kind == B200BO_ACQ_POI ||
+                          (spec->kind == B200BO_ACQ_UCB && spec->kappa >= 0.0);
+    return monotone && spec->n_gps == 1 && np_max >= kPruneMinBlocks * PBM &&
+           (m_call + PBN - 1) / PBN >= kPruneMinWaves * sm_count;
+}
+
+// screen -> pilot (first launch of a call only: tau = k-th exact key of the candidates with the k smallest bounds
+// of each screen CTA; chunks after the first keep it) -> compaction of the survivors' coordinates (so chunk
+// buffers can be reused), and on the finishing launch one gather launch over all survivors into the per-CTA lists
+// P.sel_cta (grid sm_count) that the caller merges.  No host synchronisation; the counters stay on the device.
+static int launch_pruned(b200bo_gp* g0, const PredictParams& P, int grid, bool dreg, const SelMode& sm,
+                         long long m_call, void* d_sel, cudaStream_t stream) {
+    int rc;
+    const int d = P.d, k = P.sel_k, nsm = g0->sm_count;
+    const size_t pilot_cap = (size_t)nsm * k;
+    if ((rc = g0->prune_key.reserve(sizeof(unsigned long long) * (size_t)P.m))) return rc;
+    if ((rc = g0->prune_cnt.reserve(3 * sizeof(unsigned long long)))) return rc;
+    if ((rc = g0->pilot.reserve(sizeof(double) * pilot_cap * (d + 1)))) return rc;
+    if ((rc = g0->surv.reserve(sizeof(double) * (size_t)m_call * (d + 1)))) return rc;
+    unsigned long long* cnt = g0->prune_cnt.as<unsigned long long>();
+    const GatherBuf pilot{g0->pilot.as<double>(), reinterpret_cast<long long*>(g0->pilot.as<double>() + pilot_cap * d),
+                          cnt + 1};
+    const GatherBuf surv{g0->surv.as<double>(), reinterpret_cast<long long*>(g0->surv.as<double>() + (size_t)m_call * d),
+                         cnt};
+    if (!sm.resume) CU(cudaMemsetAsync(cnt, 0, 2 * sizeof(unsigned long long), stream));
+    PredictParams S = P;
+    S.screen_key = g0->prune_key.as<unsigned long long>();
+    S.sel_resume = 0;
+    launch16<P16_SCREEN>(dreg, grid, S, stream);
+    PredictParams G = P;
+    G.m = 0;
+    G.sel_resume = 0;
+    if (!sm.resume) {
+        prune_pilot_kernel<<<grid, SEL_MAXK, 0, stream>>>(P, P.sel_cta, k, pilot);
+        G.gather_x = pilot.x;
+        G.gather_idx = pilot.idx;
+        G.gather_count = pilot.count;
+        launch16<P16_GATHER>(dreg, nsm, G, stream);
+        // the pilot's records go to d_sel only to derive tau: the final merge overwrites them
+        merge_sel_kernel<<<1, 256, 0, stream>>>(P.sel_cta, nsm, k, reinterpret_cast<SelRecord*>(d_sel));
+        prune_tau_kernel<<<1, 32, 0, stream>>>(reinterpret_cast<const SelRecord*>(d_sel), k, cnt + 2);
+        LAUNCHED();
+        LAUNCHED();
+        LAUNCHED();
+    }
+    prune_compact_kernel<<<(unsigned)((P.m + 255) / 256), 256, 0, stream>>>(S, cnt + 2, surv);
+    LAUNCHED();
+    if (sm.finish) {
+        G.gather_x = surv.x;
+        G.gather_idx = surv.idx;
+        G.gather_count = surv.count;
+        launch16<P16_GATHER>(dreg, nsm, G, stream);
+    }
+    return B200BO_OK;
+}
 
 static int eval_core(const b200bo_acq* spec, const CandSrc& src, int64_t m, double* d_acq_neg, double* d_mu,
                      double* d_sd, int k, void* d_sel, int64_t index_base, cudaStream_t stream,
@@ -1094,6 +1179,15 @@ static int eval_core(const b200bo_acq* spec, const CandSrc& src, int64_t m, doub
     if (sm.resume || !sm.finish) grid = g0->sm_count;  // chunked batches keep one list per SM across launches
     const bool small = grid > 0 && !sm.resume && sm.finish &&
                        use_small_path(m, np_max, spec->n_gps, g0->sm_count, spec->path);
+    const bool p16 = predict_impl(g0->precision) == PREDICT_IMPL_DMMA && predict_warps() == 16;
+    const long long m_call = sm.m_call ? sm.m_call : m;
+    const bool prune = !small && grid > 0 && k > 0 && p16 && !P.acq_out && !P.mu_out && !P.sd_out &&
+                       prune_eligible(spec, m_call, np_max, g0->sm_count);
+    if (!sm.resume) {
+        g0->st_screened = g0->st_full = 0;
+        g0->st_pruned = prune;
+    }
+    (prune ? g0->st_screened : g0->st_full) += m;
     bool fused_sel = false;
     if (small) {
         if (k > 0 && !P.acq_out) {  // the small path selects from the materialised values
@@ -1179,11 +1273,11 @@ static int eval_core(const b200bo_acq* spec, const CandSrc& src, int64_t m, doub
             } else {
                 predict_acq_tc_kernel<false><<<grid, PNT, kPredictSmemBytesTc, stream>>>(P);
             }
-        } else if (predict_impl(g0->precision) == PREDICT_IMPL_DMMA && predict_warps() == 16) {
-            if (dreg)
-                predict_acq16_kernel<true><<<grid, P16_NT, kPredictSmemBytesDmma, stream>>>(P);
-            else
-                predict_acq16_kernel<false><<<grid, P16_NT, kPredictSmemBytesDmma, stream>>>(P);
+        } else if (prune) {
+            if ((rc = launch_pruned(g0, P, grid, dreg, sm, m_call, d_sel, stream))) return rc;
+            grid = g0->sm_count;  // the survivors' gather launch produced the lists merged below
+        } else if (p16) {
+            launch16<P16_FULL>(dreg, grid, P, stream);
         } else if (predict_impl(g0->precision) == PREDICT_IMPL_DMMA) {
             if (dreg)
                 predict_acq_kernel<PREDICT_IMPL_DMMA, true><<<grid, PNT, kPredictSmemBytesDmma, stream>>>(P);
@@ -1195,7 +1289,7 @@ static int eval_core(const b200bo_acq* spec, const CandSrc& src, int64_t m, doub
             else
                 predict_acq_kernel<PREDICT_IMPL_DFMA, false><<<grid, PNT, kPredictSmemBytesDfma, stream>>>(P);
         }
-        LAUNCHED();
+        if (!p16) LAUNCHED();  // launch16 counts its own
         CU(cudaGetLastError());
         CU(cudaEventRecord(g0->ev1, stream));
         g_last_timed = g0;
@@ -1235,6 +1329,22 @@ extern "C" int b200bo_acq_select_philox_dev(const b200bo_acq* spec, uint64_t see
     src.lo = lo;
     src.hi = hi;
     return eval_core(spec, src, m, nullptr, nullptr, nullptr, k, d_sel, index_base, (cudaStream_t)stream_);
+}
+
+extern "C" int b200bo_last_select_stats(int64_t* screened, int64_t* evaluated) {
+    if (!screened || !evaluated) return set_err(B200BO_ERR_ARG, "NULL argument");
+    if (!g_last_timed) return set_err(B200BO_ERR_STATE, "no timed kernel on this thread");
+    const b200bo_gp* g = g_last_timed;
+    CU(cudaSetDevice(g->device));
+    CU(cudaEventSynchronize(g->ev1));
+    *screened = g->st_screened;
+    *evaluated = g->st_full;
+    if (g->st_pruned) {
+        unsigned long long c[2];
+        CU(cudaMemcpy(c, g->prune_cnt.p, sizeof(c), cudaMemcpyDeviceToHost));
+        *evaluated = (int64_t)(c[0] + c[1]);
+    }
+    return B200BO_OK;
 }
 
 extern "C" int b200bo_last_kernel_ms(float* ms) {
@@ -1295,6 +1405,7 @@ static int run_host_chunked(const b200bo_acq* spec, const double* Xc, int64_t m,
         SelMode sm;
         sm.resume = i > 0;
         sm.finish = (c0 + chunk >= m);
+        sm.m_call = m;
         if ((rc = eval_core(spec, src, mc, nullptr, nullptr, nullptr, k, g0->sel.p, c0, g0->exec_stream, sm)))
             return rc;
         CU(cudaEventRecord(g0->chunk_done[b], g0->exec_stream));

@@ -38,10 +38,17 @@ __device__ __forceinline__ void st_global_hint(double* p, double v, unsigned lon
     asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;\n" ::"l"(p), "d"(v), "l"(pol) : "memory");
 }
 
+// Modes of predict_acq16_kernel.  FULL: the fused kernel.  SCREEN: phase A in full (mu needs every K* row) but K*
+// stored for the first kScreenBlocks row blocks only, phase B over those blocks, a lower-bound key per candidate
+// (select.cuh prune_lower_bound) and per-CTA lists of the k smallest bounds.  GATHER: FULL over the candidates of a
+// gather buffer (coordinates as loaded + global index, count on the device).
+enum { P16_FULL = 0, P16_SCREEN = 1, P16_GATHER = 2 };
+constexpr int kScreenBlocks = 2;
+
 // ---- phase A: K*^T tile (np x 128) into the CTA's scratch + K* alpha_ -----------------------------
-template <bool DREG, int COV>
+template <bool DREG, int COV, int MODE>
 __device__ __forceinline__ void predict16_phase_a_impl(const PredictParams& P, const GpDev& G, long long c0,
-                                                       double* __restrict__ Ks, double* smem,
+                                                       long long m, double* __restrict__ Ks, double* smem,
                                                        double (*mu_s)[PBN], unsigned long long pol_first) {
     const int tid = threadIdx.x;
     const int d = P.d, np = G.np;
@@ -52,8 +59,8 @@ __device__ __forceinline__ void predict16_phase_a_impl(const PredictParams& P, c
         const int c = idx / d, j = idx - c * d;
         const long long gi = c0 + c;
         double v = 0.0;
-        if (gi < P.m) {
-            v = candidate_coord(P, gi, j);
+        if (gi < m) {
+            v = MODE == P16_GATHER ? P.gather_x[gi * d + j] : candidate_coord(P, gi, j);
             if (G.xform && G.xform[j] == B200BO_XFORM_ROUND) v = rint(v);
             v = v / G.ls[j];
         }
@@ -130,7 +137,7 @@ __device__ __forceinline__ void predict16_phase_a_impl(const PredictParams& P, c
                 const int n = ch * PA_CHUNK + r0 + q;
                 double kv = G.constv * cov_eval<COV>(r2[q]);
                 if (n >= G.n) kv = 0.0;
-                st_global_hint(Ks + (size_t)n * PBN + c, kv, pol_first);
+                if (MODE != P16_SCREEN || n < kScreenBlocks * PBM) st_global_hint(Ks + (size_t)n * PBN + c, kv, pol_first);
                 mu_acc = fma(al[r0 + q], kv, mu_acc);
             }
         }
@@ -142,15 +149,15 @@ __device__ __forceinline__ void predict16_phase_a_impl(const PredictParams& P, c
     __syncthreads();
 }
 
-template <bool DREG>
-__device__ __forceinline__ void predict16_phase_a(const PredictParams& P, const GpDev& G, long long c0,
+template <bool DREG, int MODE>
+__device__ __forceinline__ void predict16_phase_a(const PredictParams& P, const GpDev& G, long long c0, long long m,
                                                   double* __restrict__ Ks, double* smem, double (*mu_s)[PBN],
                                                   unsigned long long pol_first) {
     switch (cov_code(G.family, G.nu)) {
-        case 0: predict16_phase_a_impl<DREG, 0>(P, G, c0, Ks, smem, mu_s, pol_first); break;
-        case 1: predict16_phase_a_impl<DREG, 1>(P, G, c0, Ks, smem, mu_s, pol_first); break;
-        case 2: predict16_phase_a_impl<DREG, 2>(P, G, c0, Ks, smem, mu_s, pol_first); break;
-        default: predict16_phase_a_impl<DREG, 3>(P, G, c0, Ks, smem, mu_s, pol_first); break;
+        case 0: predict16_phase_a_impl<DREG, 0, MODE>(P, G, c0, m, Ks, smem, mu_s, pol_first); break;
+        case 1: predict16_phase_a_impl<DREG, 1, MODE>(P, G, c0, m, Ks, smem, mu_s, pol_first); break;
+        case 2: predict16_phase_a_impl<DREG, 2, MODE>(P, G, c0, m, Ks, smem, mu_s, pol_first); break;
+        default: predict16_phase_a_impl<DREG, 3, MODE>(P, G, c0, m, Ks, smem, mu_s, pol_first); break;
     }
 }
 
@@ -170,7 +177,8 @@ __device__ __forceinline__ void predict16_load_stage(double* as, double* bs, con
 }
 
 // ---- phase B: mma.sync m8n8k4 f64; 16 warps, warp tile 32(m) x 32(n); red[4][PBN] ----------------
-__device__ __forceinline__ void predict16_phase_b(const GpDev& G, const double* __restrict__ Ks, double* smem,
+// over the first nb row blocks of L^-1 (all np / PBM of them but in the screen)
+__device__ __forceinline__ void predict16_phase_b(const GpDev& G, const double* __restrict__ Ks, double* smem, int nb,
                                                   unsigned long long pol_last, unsigned long long pol_first) {
     constexpr int STR = PSTR_DMMA, BK = PBK_DMMA;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -185,7 +193,6 @@ __device__ __forceinline__ void predict16_phase_b(const GpDev& G, const double* 
     double csq[4][2];
 #pragma unroll
     for (int j = 0; j < 4; ++j) csq[j][0] = csq[j][1] = 0.0;
-    const int nb = np / PBM;
     for (int ib = 0; ib < nb; ++ib) {
         double acc[4][4][2];
 #pragma unroll
@@ -266,7 +273,7 @@ __device__ __forceinline__ void predict16_phase_b(const GpDev& G, const double* 
     __syncthreads();
 }
 
-template <bool DREG>
+template <bool DREG, int MODE>
 __global__ void __launch_bounds__(P16_NT, 1) predict_acq16_kernel(const PredictParams P) {
     extern __shared__ __align__(16) double smem[];
     __shared__ double mu_s[P16_SPLIT][PBN];
@@ -276,7 +283,8 @@ __global__ void __launch_bounds__(P16_NT, 1) predict_acq16_kernel(const PredictP
 
     const int tid = threadIdx.x;
     double* Ks = P.scratch + (long long)blockIdx.x * P.scratch_stride;
-    const long long ntiles = (P.m + PBN - 1) / PBN;
+    const long long m = MODE == P16_GATHER ? (long long)*P.gather_count : P.m;
+    const long long ntiles = (m + PBN - 1) / PBN;
     const unsigned long long pol_last = l2_policy_evict_last(), pol_first = l2_policy_evict_first();
     if (P.sel_cta) {
         if (tid < PBN) runsel_begin(sel_s, P.sel_cta + blockIdx.x, P.sel_resume, tid);
@@ -286,22 +294,63 @@ __global__ void __launch_bounds__(P16_NT, 1) predict_acq16_kernel(const PredictP
         const long long c0 = tile * PBN;
         for (int g = 0; g < P.n_gps; ++g) {
             const GpDev& G = P.gp[g];
-            predict16_phase_a<DREG>(P, G, c0, Ks, smem, mu_s, pol_first);
-            predict16_phase_b(G, Ks, smem, pol_last, pol_first);
+            predict16_phase_a<DREG, MODE>(P, G, c0, m, Ks, smem, mu_s, pol_first);
+            predict16_phase_b(G, Ks, smem, MODE == P16_SCREEN ? kScreenBlocks : G.np / PBM, pol_last, pol_first);
             const double* red = smem;
             if (tid < PBN) {
                 const int c = tid;
+                const bool valid = c0 + c < m;
                 const double colsq = ((red[c] + red[PBN + c]) + red[2 * PBN + c]) + red[3 * PBN + c];
                 const double mu_n = ((mu_s[0][c] + mu_s[1][c]) + mu_s[2][c]) + mu_s[3][c];
-                double val = 0.0;
-                candidate_epilogue(P, G, g, mu_n, colsq, c0 + c, base_s[c], prod_s[c], &val);
-                if (P.sel_cta && g == P.n_gps - 1)
-                    runsel_update<1>(sel_s, P.sel_k, tid, val, c0 + c + P.index_base, c0 + c < P.m);
+                if (MODE == P16_SCREEN) {  // the steps of candidate_epilogue up to sd, with the partial colsq
+                    const double mean = G.y_std * mu_n + G.y_mean;
+                    double var = G.prior - colsq;
+                    if (var < 0.0) var = 0.0;  // not fmax: a NaN must stay NaN
+                    const double lb = prune_lower_bound(P.acq_kind, mean, sqrt(var * (G.y_std * G.y_std)), P.y_max,
+                                                        P.xi, P.kappa);
+                    if (valid) P.screen_key[c0 + c] = prune_key(lb);
+                    runsel_update<1>(sel_s, P.sel_k, tid, lb, c0 + c + P.index_base, valid);
+                } else {
+                    double val = 0.0;
+                    candidate_epilogue(P, G, g, mu_n, colsq, c0 + c, base_s[c], prod_s[c], &val);
+                    if (P.sel_cta && g == P.n_gps - 1) {
+                        const long long gi = MODE == P16_GATHER ? (valid ? P.gather_idx[c0 + c] : SEL_NOIDX)
+                                                                : c0 + c + P.index_base;
+                        runsel_update<1>(sel_s, P.sel_k, tid, val, gi, valid);
+                    }
+                }
             }
             __syncthreads();
         }
     }
     if (P.sel_cta && tid < PBN) runsel_store(sel_s, P.sel_cta + blockIdx.x, tid);
+}
+
+// ---- pruned selection: gather buffers -------------------------------------------------------------
+struct GatherBuf {
+    double* x;                  // [cap][d] coordinates as phase A loads them (before transform and scaling)
+    long long* idx;             // [cap] global selection index
+    unsigned long long* count;  // appended so far
+};
+
+// append local candidate i of launch P (its device matrix or its Philox rows)
+__device__ __forceinline__ void gather_append(const PredictParams& P, long long i, const GatherBuf& B) {
+    const unsigned long long pos = atomicAdd(B.count, 1ull);
+    B.idx[pos] = i + P.index_base;
+    for (int j = 0; j < P.d; ++j) B.x[pos * P.d + j] = candidate_coord_raw(P, i, j);
+}
+
+// pilot: the candidates of the screen's per-CTA lists (k smallest lower bounds each); one block per list
+__global__ void prune_pilot_kernel(const PredictParams P, const SelList* __restrict__ lists, int k, GatherBuf B) {
+    const long long gi = threadIdx.x < k ? lists[blockIdx.x].idx[threadIdx.x] : SEL_NOIDX;
+    if (gi != SEL_NOIDX) gather_append(P, gi - P.index_base, B);
+}
+
+// survivors: every candidate whose lower-bound key is <= tau (non-strict: ties with the k-th record and its
+// lower-index rule must stay), and every candidate without a usable bound (key 0)
+__global__ void prune_compact_kernel(const PredictParams P, const unsigned long long* __restrict__ tau, GatherBuf B) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < P.m && P.screen_key[i] <= *tau) gather_append(P, i, B);
 }
 
 }  // namespace b200bo

@@ -56,19 +56,25 @@ struct PredictParams {
     double* scratch;   // gridDim.x * scratch_stride doubles
     long long scratch_stride;
     unsigned long long* clamp_count;  // nullable; [0] negative variances clamped to 0, [1] non-finite candidate coordinates
+    // pruned selection (predict16.cuh): screen output / gather-mode source
+    unsigned long long* screen_key;  // screen: [m] lower-bound selection key per candidate, 0 = must be evaluated
+    const double* gather_x;          // gather: [count][d] candidate coordinates as loaded
+    const long long* gather_idx;     // gather: [count] global selection index
+    const unsigned long long* gather_count;
 };
 
 // coordinate j of candidate gi (local index) as the reference's x_tries[gi, j]
 // A non-finite coordinate is counted in clamp_count[1]: the host entry points turn it into the ValueError
 // ("Input X contains NaN or infinity") sklearn's validate_data raises - checked where the data is read anyway instead
 // of a separate pass over the batch on the host (10 ms per 2^20 x 16 batch).
-__device__ __forceinline__ double candidate_coord(const PredictParams& P, long long gi, int j) {
-    if (P.Xc) {
-        const double v = P.Xc[gi * P.d + j];
-        if (!isfinite(v) && P.clamp_count) atomicAdd(P.clamp_count + 1, 1ull);
-        return v;
-    }
+__device__ __forceinline__ double candidate_coord_raw(const PredictParams& P, long long gi, int j) {
+    if (P.Xc) return P.Xc[gi * P.d + j];
     return philox_coord(P.seed, gi + P.index_base, j, P.pbounds[j], P.pbounds[P.d + j]);
+}
+__device__ __forceinline__ double candidate_coord(const PredictParams& P, long long gi, int j) {
+    const double v = candidate_coord_raw(P, gi, j);
+    if (P.Xc && !isfinite(v) && P.clamp_count) atomicAdd(P.clamp_count + 1, 1ull);
+    return v;
 }
 
 constexpr int PBM = 128, PBN = 128, PBK = 16, PSTAGES = 3, PNT = 256;

@@ -197,6 +197,49 @@ merge_sel_kernel(const SelList* __restrict__ lists, int nlists, int k, SelRecord
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// Pruned selection (predict16.cuh, b200bo.cu eval_core).  sigma^2 = prior - sum_i V_i^2 and every term is >= 0,
+// so the partial sum over the first row blocks of L^-1 (same per-thread / shuffle / red[] reduction tree as the
+// full sum) bounds sigma from above in floating point too: adding a non-negative number under round-to-nearest
+// never decreases a sum, and the clamp, the scaling by y_std^2 and sqrt are monotone.  mu is exact after phase A,
+// and EI, UCB (kappa >= 0) and PoI (for a < 0) increase with sigma, so the acquisition at sd_up bounds the
+// selected value val = -acq from below.  A candidate whose lower bound lies above tau, the k-th smallest exact
+// key of candidates of the same call, cannot enter the records.
+// ---------------------------------------------------------------------------------------
+// Computed EI / PoI are not monotone at the ulp level (near z << 0 the two EI terms cancel and the rounding
+// of z is amplified ~z^2 times): the bound is lowered by this relative margin of the summed magnitudes.
+constexpr double kPruneRelMargin = 9.313225746154785e-10;  // 2^-30
+constexpr double kDblMin = 2.2250738585072014e-308;
+
+// lower bound on val = -acq for a candidate with exact mean and sd <= sd_up; NaN = no usable bound (non-finite
+// intermediates, a == 0 where sd may clamp to 0 and 0/0 gives NaN, PoI with a >= 0): evaluate it in full
+__device__ __forceinline__ double prune_lower_bound(int kind, double mean, double sd_up, double y_max, double xi,
+                                                    double kappa) {
+    if (kind == B200BO_ACQ_UCB) {
+        const double v = -(mean + kappa * sd_up);  // exact bound: every operation is monotone in sd (kappa >= 0)
+        return isfinite(v) ? v : CUDART_NAN;
+    }
+    const double a = mean - y_max - xi;
+    if (!isfinite(a) || a == 0.0 || !isfinite(sd_up)) return CUDART_NAN;
+    const double z = a / sd_up;
+    const double cdf = ndtr(z);
+    if (kind == B200BO_ACQ_POI) return a < 0.0 ? -(cdf + (kPruneRelMargin * cdf + kDblMin)) : CUDART_NAN;
+    const double pdf = norm_pdf(z);
+    const double up = a * cdf + sd_up * pdf;  // the EI expression of candidate_epilogue
+    const double v = -(up + (kPruneRelMargin * (fabs(a) * cdf + sd_up * pdf) + kDblMin));
+    return isfinite(v) ? v : CUDART_NAN;
+}
+
+// screen key: 0 (below every value key) forces a full evaluation
+__device__ __forceinline__ unsigned long long prune_key(double lb) { return isnan(lb) ? 0ull : key_nan_last(lb); }
+
+// tau = key of the k-th pilot record (records as merge_sel_kernel writes them; an empty record gives the
+// all-ones key: nothing is pruned)
+__global__ void prune_tau_kernel(const SelRecord* __restrict__ rec, int k, unsigned long long* tau) {
+    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    *tau = rec[k].index < 0 ? 0xFFFFFFFFFFFFFFFFull : key_nan_last(rec[k].value);
+}
+
 // Merge of per-device record sets (multi-GPU exchange, SURVEY.md 8e): rec[g][0] = device g's argmin record
 // (NaN first), rec[g][1..k] = its top-k (ascending, index < 0 = empty).  Same ordering rules as above.
 __global__ void merge_records_kernel(const SelRecord* __restrict__ rec, int ndev, int k, SelRecord* __restrict__ out) {

@@ -255,6 +255,11 @@ int b200bo_multi_gpu_acq_eval(const b200bo_acq* specs, int n_dev, const double* 
  * device or host entry point on this thread, measured with CUDA events on its stream.
  * Synchronises on the stop event. */
 int b200bo_last_kernel_ms(float* ms);
+/* Work of the most recent fused predict+acquisition call on this thread (all chunks of a streamed host batch):
+ * *screened = candidates that went through the screen of the pruned selection (0 when the call was not
+ * pruned), *evaluated = candidates that went through the full L^-1 K*^T product (pilot + survivors when pruned,
+ * else all of them).  Synchronises on the call's stop event. */
+int b200bo_last_select_stats(int64_t* screened, int64_t* evaluated);
 
 #ifdef __cplusplus
 }
